@@ -77,7 +77,13 @@ def parse():
                     help="skip the `gpu_reference` entry (the unmodified reference modules timed on the same GPUs)")
     ap.add_argument("--gpu-ref-steps", type=int, default=10)
     ap.add_argument("--gpu-ref-precisions", default="bf16,fp16")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step computed (loss, loss centers, a seeded sample of the student "
+                         "and teacher parameters) as DIR/<name>.npy in float32")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -160,6 +166,27 @@ def synthetic_crops(batch: int, n_local: int, rank: int):
     crops = [torch.randn(batch, 3, 224, 224, generator=g) for _ in range(2)]
     crops += [torch.randn(batch, 3, 96, 96, generator=g) for _ in range(n_local)]
     return crops
+
+
+def dump_outputs(out_dir: str, loss, student, teacher, loss_mod, per_param: int = 4096) -> None:
+    """What a caller of the step holds after it: the loss, the updated loss centers and the updated student / teacher
+    parameters, one float32 .npy each.  The parameters hold ~10^8 values, so each contributes a fixed seeded sample of
+    at most `per_param` elements (all of a smaller one), concatenated in named_parameters() order; two builds run with
+    the same arguments sample the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().reshape(1), "center": loss_mod.center, "center_grid": loss_mod.center_grid}
+    for name, net in (("student_params", student), ("teacher_params", teacher)):
+        g = torch.Generator().manual_seed(0)
+        parts = []
+        for p in net.parameters():
+            flat = p.detach().reshape(-1)
+            if flat.numel() > per_param:
+                flat = flat[torch.randint(flat.numel(), (per_param,), generator=g).to(flat.device)]
+            parts.append(flat.float())
+        arrays[name] = torch.cat(parts)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def max_over_ranks(ms: float, device) -> float:
@@ -360,6 +387,8 @@ def main():
     barrier_sync()
     clocks = sampler.stop() if rank == 0 else None
     ms = max_over_ranks(e0.elapsed_time(e1), dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, l, student, teacher, loss_mod)
     launches = launches_per_step * K  # esvit_b200 kernels per step (counted in the eager steps) x K
     ms_per_step = ms / K
     value = world * B / (ms_per_step / 1e3)

@@ -32,30 +32,27 @@ SMALL = dict(img_size=112, embed_dim=32, depths=(2, 2, 2), num_heads=(1, 2, 4), 
 SMALL_W14 = dict(img_size=112, embed_dim=32, depths=(2, 2, 2), num_heads=(1, 2, 4), window_size=14)
 HEAD = dict(hidden_dim=128, bottleneck_dim=64)
 K = 384
+INIT_SEED = 0
 HP = dict(lr=5e-4, weight_decay=0.04, clip_grad=3.0, freeze_last_layer=1, momentum_teacher=0.996,
           teacher_temp=0.04, student_temp=0.1, center_momentum=0.9)
 
 
-def build(dense: bool, seed: int = 0, small=None):
+def build(dense: bool, small=None):
+    """The reference's own modules, initialised with the seeded weights of ST.synthetic_state_dict (the fixture stores
+    the seed and the layout, not the weights)."""
     ns = R.load()
     spec = S.SwinSpec(use_dense_prediction=dense, **(small or SMALL))
-    m = R.build_swin(spec, K, seed=seed)
-    torch.manual_seed(seed + 1)
+    m = R.build_swin(spec, K)
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
         m.head = ns.DINOHead(m.num_features, K, **HEAD)
         if dense:
             m.head_dense = ns.DINOHead(m.num_features, K, **HEAD)
-    # random (not zero / one) biases, LN affine and bias tables so every term is exercised
-    g = torch.Generator().manual_seed(seed + 2)
-    with torch.no_grad():
-        for n, p in m.named_parameters():
-            if n.endswith(".bias"):
-                p.copy_(torch.randn(p.shape, generator=g) * 0.05)
-            elif p.dim() == 1 and "norm" in n:
-                p.copy_(1 + torch.randn(p.shape, generator=g) * 0.1)
-            elif "relative_position_bias_table" in n:
-                p.copy_(torch.randn(p.shape, generator=g) * 0.5)
+    ref = m.state_dict()
+    sd = ST.synthetic_state_dict([(k, tuple(v.shape)) for k, v in ref.items()], INIT_SEED)
+    for k, v in ref.items():
+        assert sd[k].dtype == v.dtype and (v.dtype.is_floating_point or torch.equal(sd[k], v)), k
+    m.load_state_dict(sd)
     return ns, spec, m
 
 
@@ -98,8 +95,9 @@ def stats(d):
 
 
 def make(dense: bool, sd_init=None, small=None, compact: bool = False):
-    """compact: keep the initial state_dict, losses, gradient / parameter statistics and a few full gradients only (the
-    crops are regenerated from their seed)."""
+    """The fixture keeps the seeds and the layout of the inputs (crops and weights are regenerated from them), losses,
+    centers, sums and norms of every gradient / parameter / output and a seeded sample of the elements of a few of them.
+    compact: no teacher outputs or region-match indices."""
     small = small or SMALL
     R.ensure_process_group()
     ns, spec, student = build(dense, small=small)
@@ -141,30 +139,29 @@ def make(dense: bool, sd_init=None, small=None, compact: bool = False):
     assert torch.allclose(orc.center, loss_mod.center, atol=1e-6)
 
     r0 = rec[0]
+    so, to = r0["student_output"], r0["teacher_output"]
+    outputs = dict(s_cls=so[0], s_region=so[1], s_fea=so[2]) if dense else dict(s_out=so, t_out=to)
+    if dense and not compact:
+        outputs.update(t_cls=to[0], t_region=to[1], t_fea=to[2])
+    outputs = {k: v.detach() for k, v in outputs.items()}
     out = dict(
         meta=dict(spec=dict(small, use_dense_prediction=dense), head=HEAD, out_dim=K, batch=B,
                   n_local=n_local if dense else 0, ncrops=ncrops, hp=HP, nsteps=nsteps,
                   crop_seed=1234, global_size=112, local_size=48,
+                  init_seed=INIT_SEED, layout=[(k, tuple(v.shape)) for k, v in sd0.items()],
                   generator="oracle/make_golden.py (reference run on CPU fp32, torch %s)" % torch.__version__),
         losses=[r["loss"] for r in rec], center_after=loss_mod.center.clone(),
         final_student_stats=stats({k: sd_s[k] for k in orc.names}),
         final_teacher_stats=stats({k: sd_t[k] for k in orc.names}),
-        final_teacher_full={k: sd_t[k].clone() for k in FULL_GRADS if k in sd_t},
+        final_teacher_sample={k: ST.sample_elements(sd_t[k]) for k in FULL_GRADS if k in sd_t},
         grads_step0_stats=stats(r0["grads"]),
-        grads_step0_full={k: r0["grads"][k] for k in FULL_GRADS if k in r0["grads"]},
+        grads_step0_sample={k: ST.sample_elements(r0["grads"][k]) for k in FULL_GRADS if k in r0["grads"]},
+        out_stats=stats(outputs), out_sample={k: ST.sample_elements(v) for k, v in outputs.items()},
     )
-    if compact:
-        so = r0["student_output"]
-        out.update(state_dict={k: v for k, v in sd0.items() if v.dtype.is_floating_point},  # index buffers = closed forms
-                   s_cls_stats=stats(dict(s_cls=so[0].detach(), s_region=so[1].detach(), s_fea=so[2].detach())),
-                   s_npatch=list(so[3]))
-        return out
     if dense:
-        out.update(state_dict=sd0, crops=crops)
-        so, to = r0["student_output"], r0["teacher_output"]
-        out.update(s_cls=so[0].detach(), s_region=so[1].detach(), s_fea=so[2].detach(), s_npatch=list(so[3]),
-                   t_cls=to[0].detach(), t_region=to[1].detach(), t_fea=to[2].detach(), t_npatch=list(to[3]),
-                   center_grid_after=loss_mod.center_grid.clone())
+        out["s_npatch"] = list(so[3])
+    if dense and not compact:
+        out.update(t_npatch=list(to[3]), center_grid_after=loss_mod.center_grid.clone())
         # argmax indices of the first step, recomputed with the reference's own expression (main_esvit.py:735-736)
         Bn, N = B, to[3][0]
         split = [so[3][0]] * 2 + [so[3][1]] * (ncrops - 2)
@@ -181,8 +178,6 @@ def make(dense: bool, sd_init=None, small=None, compact: bool = False):
                 assert torch.equal(idx[(iq, v)], orc.indices_step[(iq, v)])
         out["indices"] = idx
         assert torch.allclose(orc.center_grid, loss_mod.center_grid, atol=1e-6)
-    else:
-        out.update(s_out=r0["student_output"].detach(), t_out=r0["teacher_output"].detach())
     return out
 
 
@@ -190,7 +185,7 @@ if __name__ == "__main__":
     if not R.available():
         sys.exit("reference tree not found; golden vectors can only be generated in the build container")
     dense = make(True)
-    view = make(False, dense["state_dict"])
+    view = make(False, ST.synthetic_state_dict(dense["meta"]["layout"], INIT_SEED))
     os.makedirs(OUT, exist_ok=True)
     path = os.path.join(OUT, "esvit_small.pt")
     torch.save(dict(dense=dense, view=view), path)

@@ -8,8 +8,9 @@ modelled by an optional ``all_reduce`` hook for the gloo tests.
 """
 from __future__ import annotations
 
+import math
 import time
-from typing import Callable, Dict, List, Optional
+from typing import Callable, Dict, List, Optional, Tuple
 
 import torch
 
@@ -102,6 +103,38 @@ def synthetic_crops(batch: int, n_local: int, seed: int = 1234, global_size: int
     crops = [torch.randn(batch, 3, global_size, global_size, generator=g) for _ in range(2)]
     crops += [torch.randn(batch, 3, local_size, local_size, generator=g) for _ in range(n_local)]
     return [c.to(device) for c in crops]
+
+
+def synthetic_state_dict(layout: List[Tuple[str, Tuple[int, ...]]], seed: int) -> Dict[str, Tensor]:
+    """Seeded fp32 weights for the (name, shape) layout of a reference state_dict, so that a fixture stores a seed and
+    a layout instead of the weights.  Random (not zero / one) biases, LN affine and bias tables exercise every term;
+    Linear / conv weights follow the reference's trunc_normal_(std=.02) scale; DINOHead's frozen weight_g is 1
+    (models/vision_transformer.py DINOHead); relative_position_index is its closed form."""
+    g = torch.Generator().manual_seed(seed)
+    sd = {}
+    for name, shape in layout:
+        shape = tuple(shape)
+        if name.endswith("relative_position_index"):
+            sd[name] = S.rel_pos_index(math.isqrt(shape[0]))
+        elif name.endswith("last_layer.weight_g"):
+            sd[name] = torch.ones(shape)
+        elif name.endswith(".bias"):
+            sd[name] = torch.randn(shape, generator=g) * 0.05
+        elif len(shape) == 1 and "norm" in name:
+            sd[name] = 1 + torch.randn(shape, generator=g) * 0.1
+        elif "relative_position_bias_table" in name:
+            sd[name] = torch.randn(shape, generator=g) * 0.5
+        else:
+            sd[name] = torch.randn(shape, generator=g) * 0.02
+    return sd
+
+
+def sample_elements(t: Tensor, n: int = 512, seed: int = 0) -> Tensor:
+    """A fixed, seeded choice of n elements of t (all of them, permuted, when t is smaller): what a fixture stores of a
+    tensor too large to keep whole, and what a test takes of its own result to compare with it."""
+    flat = t.detach().reshape(-1)
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(seed))[:n]
+    return flat[idx.to(flat.device)]
 
 
 def time_steps(stepper: OracleStep, crops: List[Tensor], steps: int, warmup: int) -> float:

@@ -2,6 +2,9 @@ import os
 
 import torch
 
+from oracle import step as ST
+from oracle import swin as S
+
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "esvit_small.pt")
 
 
@@ -16,8 +19,67 @@ def assert_close(a, b, tol, name=""):
     assert r < tol, f"{name}: rel l2 error {r:.3e} >= {tol:.1e}"
 
 
+def assert_matches_sample(t, sample, atol, rtol, name=""):
+    """t agrees elementwise with a fixture's seeded sample of the reference's tensor (oracle.step.sample_elements)."""
+    got = ST.sample_elements(t.detach().cpu())
+    assert torch.allclose(got, sample, atol=atol, rtol=rtol), (name, float((got - sample).abs().max()))
+
+
+def assert_matches_stats(t, stats, tol, name=""):
+    """sum and norm of t against the (sum, norm) a fixture stores for the reference's tensor."""
+    ssum, nrm = stats
+    t = t.detach().double().cpu()
+    assert abs(float(t.norm()) - nrm) < tol * nrm + 1e-9, (name, float(t.norm()), nrm)
+    assert abs(float(t.sum()) - ssum) < tol * nrm * t.numel() ** 0.5 + 1e-9, (name, float(t.sum()), ssum)
+
+
+def load_fixture(name: str = "esvit_small.pt"):
+    """A fixture of tests/golden with its seeded inputs regenerated: dense["state_dict"] and dense["crops"]."""
+    G = torch.load(os.path.join(os.path.dirname(GOLDEN), name), map_location="cpu", weights_only=False)
+    M = G["dense"]["meta"]
+    G["dense"]["state_dict"] = ST.synthetic_state_dict(M["layout"], M["init_seed"])
+    G["dense"]["crops"] = ST.synthetic_crops(M["batch"], M["n_local"], seed=M["crop_seed"], global_size=M["global_size"],
+                                             local_size=M["local_size"])
+    return G
+
+
+_golden = {}
+
+
 def load_golden():
-    return torch.load(GOLDEN, map_location="cpu", weights_only=False)
+    """esvit_small.pt with whole tensors where the fixture keeps a sample of the reference's: the forward outputs,
+    region-match indices, step-0 gradients and final teacher weights of the CPU oracle on the fixture's inputs, each
+    checked here against the reference's sample, stats and losses (tests/test_oracle_golden.py checks the same)."""
+    if "G" in _golden:
+        return _golden["G"]
+    G = load_fixture()
+    for which in ("dense", "view"):
+        dense = which == "dense"
+        D, M = G[which], G[which]["meta"]
+        sd = {k: v for k, v in G["dense"]["state_dict"].items() if dense or not k.startswith("head_dense")}
+        crops = G["dense"]["crops"][:M["ncrops"]]
+        spec = S.SwinSpec(**dict(G["dense"]["meta"]["spec"], use_dense_prediction=dense))
+        orc = ST.OracleStep(sd, spec, M["ncrops"], M["out_dim"], **M["hp"])
+        losses = [orc.step(crops, epoch=0, keep_grads=(i == 0)) for i in range(M["nsteps"])]
+        for a, b in zip(losses, D["losses"]):
+            assert abs(a - b) < 2e-5 * max(1.0, abs(b)), (which, losses, D["losses"])
+        D["grads_step0_full"] = {k: orc.grads_step[k] for k in D["grads_step0_sample"]}
+        D["final_teacher_full"] = {k: orc.teacher[k].detach() for k in D["final_teacher_sample"]}
+        for k, g in D["grads_step0_sample"].items():
+            assert_matches_sample(D["grads_step0_full"][k], g, 1e-7 + 1e-4 * float(g.abs().max()), 1e-3, k)
+        for k, v in D["final_teacher_sample"].items():
+            assert_matches_sample(D["final_teacher_full"][k], v, 1e-5, 0.0, k)
+        if dense:
+            with torch.no_grad():
+                s = S.multicrop_forward(crops, sd, spec)
+                t = S.multicrop_forward(crops[:2], sd, spec)
+            D.update(s_cls=s[0], s_region=s[1], s_fea=s[2], t_cls=t[0], t_region=t[1], t_fea=t[2])
+            for k, v in D["out_sample"].items():
+                assert_matches_sample(D[k], v, 2e-5, 1e-4, k)
+            for key, ref in D["indices"].items():
+                assert torch.equal(orc.indices_step[key], ref), key
+    _golden["G"] = G
+    return G
 
 
 # tolerances (documented in DESIGN.md §parity): the CUDA path runs its GEMMs and branch activations in bf16
